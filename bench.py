@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            (N>1 via torch.distributed.run, one rank per GPU)
   python bench.py --impl reference ...                     (CPU arm: one worker per host core over the same files)
   python bench.py --workload scan_agg|join|sort_shuffle|all   (default all: the headline + the other configs as sub-results)
+  python bench.py --dump-outputs DIR ...                   (also write every leg's last timed result as DIR/<leg>.<column>.npy)
 
 Headline (`metric`, `value`, `e2e`, `roofline`): BASELINE configs[1] -- ParquetScan -> Filter -> HashAggregate (GROUP BY int64,
 SUM/COUNT) over a synthetic TPC-DS SF100 `store_sales` (287,997,024 rows); one step = one pass of the whole plan.
@@ -34,6 +35,7 @@ import pyarrow.parquet as pq
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the bench writes nothing into the source tree, which may be read-only
 
 SF100_ROWS = 287_997_024
 ROWS_PER_FILE = 16_000_000
@@ -54,7 +56,10 @@ def gen_file(path: str, rows: int, seed: int):
         "ss_sold_date_sk": pa.array(rng.integers(DATE_LO, DATE_HI, rows, dtype=np.int32), mask=rng.random(rows) < 0.04),
     }, schema=SCHEMA)
     # Spark's writer defaults: SNAPPY pages, dictionary encoding, ~128 MB row groups (8M rows x 3 projected columns)
-    pq.write_table(t, path, compression=CODEC, use_dictionary=True, row_group_size=8_000_000, data_page_size=1 << 20)
+    # written under a temporary name and renamed: a run that dies mid-write leaves no partial file for later runs to reuse as input
+    tmp = f"{path}.{os.getpid()}.tmp"
+    pq.write_table(t, tmp, compression=CODEC, use_dictionary=True, row_group_size=8_000_000, data_page_size=1 << 20)
+    os.replace(tmp, path)
 
 
 def gen_dataset(directory: str, total_rows: int) -> list[tuple[str, int]]:
@@ -241,6 +246,20 @@ def do_workload(args, w: str) -> bool:
     return args.workload in ("all", w)
 
 
+def dump_outputs(directory: str, outputs: dict[str, pa.Table]):
+    """--dump-outputs: every column of every leg's last timed result as <directory>/<leg>.<column>.npy in float64 (NULL is NaN,
+    decimals by value).  Rows are sorted by all columns: the engine's row order is unspecified, the rows are what two builds must agree on.
+    A column whose name is empty or repeated (the state columns of a PARTIAL aggregate) is named col<position>."""
+    os.makedirs(directory, exist_ok=True)
+    for leg, t in outputs.items():
+        names = t.column_names
+        t = t.rename_columns([n if n and names.count(n) == 1 else f"col{i}" for i, n in enumerate(names)])
+        if t.num_rows:
+            t = t.take(pc.sort_indices(t, sort_keys=[(n, "ascending") for n in t.column_names], null_placement="at_start"))
+        for name, col in zip(t.column_names, t.columns):
+            np.save(os.path.join(directory, f"{leg}.{name}.npy"), pc.cast(col, pa.float64()).to_numpy().astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -250,9 +269,14 @@ def main():
     ap.add_argument("--workload", default="all", choices=["all", "scan_agg", "join", "sort_shuffle"])
     ap.add_argument("--rows", type=int, default=SF100_ROWS)
     ap.add_argument("--op-rows", type=int, default=int(os.environ.get("AURON_BENCH_OP_ROWS", 64_000_000)), help="rows per GPU of the sort/shuffle workload")
-    ap.add_argument("--data-dir", default=os.path.join(tempfile.gettempdir(), "auron_b200_bench"))
+    # per user: on a shared host another user's directory of the same name is not writable
+    ap.add_argument("--data-dir", default=os.path.join(tempfile.gettempdir(), f"auron_b200_bench_{os.getuid()}"))
     ap.add_argument("--skip-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the result arrays of the last timed step of every GPU leg "
+                                                          "as DIR/<leg>.<column name or col<position>>.npy (float64, rows in a canonical order; rank 0's results when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -277,7 +301,7 @@ def main():
         for _ in range(warm):
             arm.run()
         rows, secs = 0, 0.0
-        steps = max(1, min(args.steps, 3))               # every step is the WHOLE table (all files) at least once: bounded to a few of them
+        steps = args.steps                               # every step is the WHOLE table (all files) at least once
         for _ in range(steps):
             r, s = arm.run()
             rows += r
@@ -400,7 +424,9 @@ def main():
                             "how": "the same kernel timed by the same events in extra untimed steps with one batch in flight at a time (AURON_FUSED_ONE_LANE=1)"}
         return res
 
-    ctx = dict(args=args, torch=torch, dist=dist, P=P, runtime=runtime, timed=timed, roofline_of=roofline_of, world=world, rank=rank, local_rank=local_rank, cores=cores)
+    outputs: dict[str, pa.Table] = {}      # leg -> result of its last timed step (--dump-outputs)
+    ctx = dict(args=args, torch=torch, dist=dist, P=P, runtime=runtime, timed=timed, roofline_of=roofline_of, world=world, rank=rank, local_rank=local_rank, cores=cores,
+               outputs=outputs)
     do = (lambda w: do_workload(args, w))
     line = None
 
@@ -451,6 +477,7 @@ def main():
         with ClockSampler(local_rank) as cs:
             dt, kern, out, value_spread = timed(mk(plan_hbm), args.steps, True)
         clocks = cs.summary()
+        outputs["scan_agg"] = out
         value = world * total_rows * args.steps / dt
         os.environ["AURON_FUSED_ONE_LANE"] = "1"      # two untimed steps without overlap between batches: the kernels' own durations
         _, kern_alone, _, _ = timed(mk(plan_hbm), 2, True)
@@ -464,6 +491,7 @@ def main():
             plan_host = build_plan(P, paths, sizes)
             timed(mk(plan_host), max(1, min(args.warmup, 2)), False)
             dtf, _, out_f, sp = timed(mk(plan_host), args.steps, False)
+            outputs["scan_agg_e2e"] = out_f
             e2e = {"value": world * total_rows * args.steps / dtf, "unit": "rows/s", "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": out_f.nbytes,
                    "ms_per_step": 1000 * dtf / args.steps, "step_ms": sp,
                    "input": "parquet files read by the engine (OS page cache -> pread into pinned staging -> H2D): the path a JVM host drives"}
@@ -478,6 +506,7 @@ def main():
             plan_pin = build_plan(P, pin_paths, sizes)
             timed(mk(plan_pin), 1, False)
             dte, _, out_e, sp = timed(mk(plan_pin), args.steps, False)
+            outputs["scan_agg_e2e_pinned"] = out_e
             e2e["pinned_images"] = {"value": world * total_rows * args.steps / dte, "ms_per_step": 1000 * dte / args.steps, "step_ms": sp,
                                     "input": "parquet file images registered in pinned host memory (auron_b200_put_host_file): H2D per column chunk, no pread"}
             for hp in pin_paths:
@@ -519,10 +548,12 @@ def main():
     else:
         line["workloads"] = workloads
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
 
 # ================================================================================================ config 3: HashJoin store_sales x date_dim
-def bench_join(args, torch, dist, P, runtime, timed, roofline_of, world, rank, local_rank, cores):
+def bench_join(args, torch, dist, P, runtime, timed, roofline_of, world, rank, local_rank, cores, outputs):
     """BASELINE configs[2]: inner hash join, build = date_dim (73,049 rows: d_date_sk int32, d_year int32), probe = store_sales SF100
     (287,997,024 rows: ss_sold_date_sk int32 drawn from a ~1,800-day window, 4 % NULL; payload ss_ext_sales_price decimal(7,2)).  The joined
     rows stay on the device: a global SUM/COUNT over them is the result that leaves (so the measurement is the join, not a 6 GB D2H)."""
@@ -549,11 +580,12 @@ def bench_join(args, torch, dist, P, runtime, timed, roofline_of, world, rank, l
         return P.task_definition(P.agg(j, [], [], [P.agg_expr("SUM", [P.col("d_year")], pa.int64()), P.agg_expr("SUM", [P.col("ss_ext_sales_price")], pa.decimal128(17, 2)),
                                                    P.agg_expr("COUNT", [P.col("ss_sold_date_sk")], pa.int64())], ["y", "p", "c"], ["PARTIAL"] * 3))
 
-    steps, warm = max(2, args.steps // 2), max(1, min(args.warmup, 2))
+    steps, warm = args.steps, max(1, min(args.warmup, 2))
     td = plan(rid_ss, rid_dd)
     mk = lambda: runtime.Task(td, device=local_rank)
     timed(mk, warm, False)
     dt, kern, out, spread = timed(mk, steps, True)
+    outputs["join"] = out
     matched = int((~null).sum())
     exp_year = int(dyear[sold[~null] - 2415022].astype(np.int64).sum())
     ok = out.column(2)[0].as_py() == matched and out.column(0)[0].as_py() == exp_year
@@ -564,6 +596,7 @@ def bench_join(args, torch, dist, P, runtime, timed, roofline_of, world, rank, l
         mkh = lambda: runtime.Task(td_h, {"host_ss": ss.to_batches(max_chunksize=chunk), "host_dd": dd.to_batches()}, device=local_rank)
         timed(mkh, 1, False)
         dth, _, outh, sp = timed(mkh, steps, False)
+        outputs["join_e2e"] = outh
         e2e = {"value": world * n * steps / dth, "unit": "rows/s", "h2d_bytes_per_step": ss.nbytes + dd.nbytes, "d2h_bytes_per_step": outh.nbytes,
                "ms_per_step": 1000 * dth / steps, "step_ms": sp, "input": "Arrow batches in pinned host memory exported through the FFI reader (24M-row batches)"}
     alg = {"join_probe": n * 4 + n // 8 + matched * 8,        # probe keys + validity in, (probe row, build row) pairs out
@@ -589,7 +622,7 @@ def bench_join(args, torch, dist, P, runtime, timed, roofline_of, world, rank, l
 
 
 # ================================================================================================ config 4: SortExec + ShuffleWriterExec
-def bench_sort_shuffle(args, torch, dist, P, runtime, timed, roofline_of, world, rank, local_rank, cores):
+def bench_sort_shuffle(args, torch, dist, P, runtime, timed, roofline_of, world, rank, local_rank, cores, outputs):
     """BASELINE configs[3]: every GPU holds a shard of store_sales projected to (ss_item_sk int32, ss_ticket_number int64, ss_ext_sales_price
     decimal(7,2)) = 28 B/row.  Leg 1: SortExec ORDER BY ss_item_sk.  Leg 2: ShuffleWriterExec hash(ss_item_sk) into 200 Spark partitions --
     N = 1: Auron's compacted shuffle format (.data + .index) written to tmpfs; N > 1: the hash repartition is exchanged between the GPUs
@@ -605,7 +638,7 @@ def bench_sort_shuffle(args, torch, dist, P, runtime, timed, roofline_of, world,
     rid = f"bs_t4_{rank}"
     for b in t4.to_batches(max_chunksize=16_000_000):
         runtime.put_device_batch(rid, b, device=local_rank)
-    steps, warm = max(2, args.steps // 2), max(1, min(args.warmup, 2))
+    steps, warm = args.steps, max(1, min(args.warmup, 2))
     res = {"steps": steps,
            "config": {"workload": "BASELINE configs[3]: SortExec + ShuffleWriterExec hash(ss_item_sk) -> 200 partitions, store_sales projected to 28 B/row",
                       "rows_per_gpu": n, "full_share_rows_per_gpu_at_sf1000_8gpu": 359_998_500, "partitions": 200,
@@ -616,18 +649,17 @@ def bench_sort_shuffle(args, torch, dist, P, runtime, timed, roofline_of, world,
     mk = lambda: runtime.Task(td_sort, device=local_rank)
     timed(mk, warm, False)
     dt, kern, out, spread = timed(mk, steps, True)
+    outputs["sort"] = out
     res["sort"] = {"value": world * n * steps / dt, "unit": "rows/s", "ms_per_step": 1000 * dt / steps, "step_ms": spread,
                    "roofline": roofline_of(kern, steps, dt, {"radix_sort": 3 * 2 * 12 * n, "take": 2 * 28 * n}), "result_ok": out.column(0)[0].as_py() == n}
     # ---- leg 2: shuffle write / exchange
     if world == 1:
-        d = "/dev/shm/auron_bench_shuffle"
-        os.makedirs(d, exist_ok=True)
+        # a directory of this run's own on tmpfs: on a shared host a fixed path may belong to another user
+        d = tempfile.mkdtemp(prefix="auron_bench_shuffle_", dir="/dev/shm" if os.path.isdir("/dev/shm") else None)
         # every map task writes its own new .data / .index pair (as in Spark): rewriting one path would charge the release of the old
         # file's pages to the step
-        import glob
         import itertools
-        for f in glob.glob(f"{d}/s*"):
-            os.remove(f)
+        import shutil
         serial = itertools.count()
 
         def mk():
@@ -635,11 +667,14 @@ def bench_sort_shuffle(args, torch, dist, P, runtime, timed, roofline_of, world,
             return runtime.Task(P.task_definition(P.shuffle_writer(P.ffi_reader(t4.schema, rid), P.hash_repartition([P.col("ss_item_sk")], 200),
                                                                    f"{d}/s{k}.data", f"{d}/s{k}.index")), device=local_rank)
 
-        timed(mk, warm, False)
-        dt, kern, out, spread = timed(mk, steps, True)
-        fsz = os.path.getsize(f"{d}/s0.data")
-        for f in glob.glob(f"{d}/s*"):
-            os.remove(f)
+        try:
+            timed(mk, warm, False)
+            dt, kern, out, spread = timed(mk, steps, True)
+            fsz = os.path.getsize(f"{d}/s0.data")
+            with open(f"{d}/s{next(serial) - 1}.index", "rb") as fh:          # the .index of the last timed step: per-partition byte offsets
+                outputs["shuffle"] = pa.table({"index_offsets": np.frombuffer(fh.read(), dtype="<i8")})
+        finally:
+            shutil.rmtree(d)
         res["shuffle"] = {"value": n * steps / dt, "unit": "rows/s", "ms_per_step": 1000 * dt / steps, "step_ms": spread, "file_bytes": fsz,
                           "file_gbs": fsz * steps / dt / 1e9, "mode": "ShuffleWriterExec -> .data/.index on tmpfs (LZ4 frames, Auron compacted format)",
                           "roofline": roofline_of(kern, steps, dt, {"murmur3_partition_ids": 8 * n, "partition_rows": 8 * n, "take": 2 * 28 * n, "serde_write": 2 * 28 * n,
@@ -654,6 +689,7 @@ def bench_sort_shuffle(args, torch, dist, P, runtime, timed, roofline_of, world,
         mk = lambda: runtime.Task(td_x, device=local_rank)
         timed(mk, warm, False)
         dt, kern, out, spread = timed(mk, steps, True)
+        outputs["shuffle"] = out
         cnt = torch.tensor([out.column(0)[0].as_py(), out.column(1)[0].as_py(), int(ticket.sum())], device="cuda", dtype=torch.int64)
         dist.all_reduce(cnt)
         comm = n * 28 * (world - 1) // world            # bytes this rank sends (= receives) per step

@@ -29,12 +29,11 @@ def _run(plan, is_task_definition=False):
         return pa.Table.from_batches(list(task), schema=task.schema)
 
 
-def test_config2_full_size_checksums(tmp_path_factory):
+def test_config2_full_size_checksums(tmp_path):
     # ParquetScan -> Filter -> HashAggregate over all 287,997,024 rows (SNAPPY pages), checked against numpy reductions of
-    # the very arrays the files were written from (regenerated from the same seeds)
-    import tempfile
-    d = os.path.join(tempfile.gettempdir(), "auron_b200_bench")               # shared with bench.py: generated once per box
-    files = bench.gen_dataset(d, SF100)
+    # the very arrays the files were written from (regenerated from the same seeds).  The files are written here, never taken
+    # from a directory an earlier run left behind.
+    files = bench.gen_dataset(str(tmp_path), SF100)
     paths = [f for f, _ in files]
     exp_cnt = exp_sum = 0
     seen = np.zeros(bench.N_ITEMS + 1, dtype=bool)
@@ -55,6 +54,8 @@ def test_config2_full_size_checksums(tmp_path_factory):
         cnt_g += np.bincount(item[sel], minlength=bench.N_ITEMS + 1)
         sum_g += np.bincount(item[sel], weights=qty[sel].astype(np.float64), minlength=bench.N_ITEMS + 1).astype(np.int64)   # exact: < 2^53
     out = _run(bench.build_plan(P, paths, [os.path.getsize(p) for p in paths]), is_task_definition=True)
+    for p in paths:                                                         # ~1.4 GB: not kept for pytest's retained temp dirs
+        os.remove(p)
     assert out.num_rows == int(seen.sum())                                  # every selected item is a group, exactly once
     assert len(set(out.column(0).to_pylist())) == out.num_rows
     assert int(out.column(2).to_numpy().sum()) == exp_cnt                   # COUNT(ss_quantity)
